@@ -273,6 +273,29 @@ def gemm_traffic():
         return dict(bytes=None, note=f"profiles/{name} missing")
 
 
+DUMP_SAMPLE = 65536   # elements kept per weight matrix by --dump-outputs
+
+
+def dump_outputs(out_dir: str, e, loss: float, grad_norm: float):
+    """What the last timed step returns to its caller: loss and grad-norm, and the fp32 master weights it
+    updated -- of the first and last decoder layers and every tensor outside the layers (embedding, final
+    norm, lm_head). A matrix is kept as DUMP_SAMPLE elements at fixed seeded flat indices, a vector whole:
+    4.3 MB in all at Llama-2-7B size. Each array goes to out_dir/<name>.npy."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.float64(loss))
+    np.save(os.path.join(out_dir, "grad_norm.npy"), np.float64(grad_norm))
+    keep = (".layers.0.", f".layers.{e.arch.num_layers - 1}.")
+    for i, (name, shape) in enumerate(e.params()):
+        if ".layers." in name and not any(k in name for k in keep):
+            continue
+        w = e.read_state(name, shape, "master").reshape(-1)
+        if len(shape) > 1 and w.size > DUMP_SAMPLE:
+            w = w[np.sort(np.random.default_rng(i).choice(w.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), w)
+
+
 def workload_config(n_gpus: int):
     return dict(workload="Llama-2-7B bf16 causal-LM fine-tune, seq 4096 (BASELINE.json configs[1])",
                 global_batch=PER_DEVICE_BATCH * n_gpus, seq_len=4096, per_device_batch=PER_DEVICE_BATCH,
@@ -383,6 +406,8 @@ def run_ours(args):
     launches = e.launch_count() - launches0
     loss_res, gn_res = e.read_scalars()
     require_finite("resident timed region", loss_res, gn_res)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, e, loss_res, gn_res)
 
     # ---- timed region 2: end to end through the host-buffer API ----
     barrier()
@@ -571,7 +596,12 @@ def main():
     ap.add_argument("--shard-state", action="store_true", default=bool(os.environ.get("B200W_SHARD_STATE")),
                     help="N>1: fp32 master / Adam moments sharded over the ranks (reduce-scatter + all-gather)")
     ap.add_argument("--decode-only", action="store_true", help="run only the decode leg and print its object")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed fine-tune step computed (loss, grad-norm, sampled updated "
+                         "weights) as DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.decode_only):
+        ap.error("--dump-outputs writes the outputs of the CUDA fine-tune step (--impl ours, not --decode-only)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     MICRO_BATCH = args.micro_batch
     RECOMPUTE = bool(args.recompute)

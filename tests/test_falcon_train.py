@@ -52,8 +52,7 @@ def test_falcon_forward_logits():
     fx, oa, arch, params = _load()
     e = _engine(arch, params, 2)
     logits, nll, _ = e.forward(fx["ids"], fx["labels"])
-    gold = fx["logits"].reshape(-1, oa.vocab_size)
-    err = rel_err(logits, gold)
+    err = rel_err(logits.reshape(-1)[::int(fx["logits_stride"])], fx["logits_sample"])
     print(f"falcon: logits rel_err {err:.3e}")
     assert err < 1.5e-2
     e.close()
